@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- FM-SGD examples/sec on synthetic Criteo-shaped CSR minibatches (BASELINE.json).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 One "step" = one minibatch through the whole hot path of SGDLearner::IterateData
@@ -17,6 +17,9 @@ Printed JSON line (rank 0):
   roofline     dominant kernel (fused FM forward+backward): algorithmic bytes / event-timed
                duration vs the measured HBM peak in MEASURED_PEAKS.json
   cpu_baseline the reference's own CPU SGD path (oracle/_ref) on a bounded sample, host cores
+
+--dump-outputs DIR (one GPU) writes what the timed steps left behind as DIR/<name>.npy, so that two builds can be
+compared output for output on the same seeded inputs (see dump_outputs).
 """
 import argparse
 import json
@@ -55,6 +58,9 @@ def parse_args():
     ap.add_argument("--cpu-rows", type=int, default=0,
                     help="rows per CPU batch (0: 4096 for the in-run cpu_baseline sample, the full batch for --impl reference)")
     ap.add_argument("--engine-kw", default="", help="extra engine kwargs k=v,k=v (tuning experiments)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the model entries of a seeded sample of the last batch's keys "
+                         "and the progress counters as DIR/<name>.npy (one GPU only)")
     return ap.parse_args()
 
 
@@ -313,6 +319,31 @@ def gen_raw_set(args, nb, seed0, torch, rows=None):
     return out
 
 
+DUMP_MAX_BYTES = 64 << 20
+DUMP_MAX_KEYS = 1 << 16
+
+
+def dump_outputs(E, d, args, last_batch, prog):
+    """what a caller of the timed path receives after its last step, as float arrays in d/<name>.npy:
+       progress                  [loss, penalty, auc, nnz_w, nrows] of dfb_read_progress, summed over the warm-up and
+                                 timed steps
+       fea_cnt, w, sqrt_g, z     per key, the model entry after the last step (dfb_read_entries) ...
+       has_V, V, V_cg            ... for a fixed, seeded sample of the distinct keys of the last timed batch (ascending
+                                 reversed keys; every one of them was updated by that step).  has_V: 1 V row, 0 none.
+    The sample is bounded so that all files together stay under DUMP_MAX_BYTES."""
+    _, keys, _ = localize_np(last_batch["ids"].numpy().view(np.uint64))
+    k = args.vdim
+    n = min(len(keys), DUMP_MAX_KEYS, (DUMP_MAX_BYTES - (1 << 16)) // (4 * (5 + 2 * k)))
+    sel = np.sort(np.random.default_rng(0).choice(len(keys), n, replace=False))
+    scal, hasv, V, cg = E.read_entries(keys[sel])
+    arrays = {"progress": np.array([prog.loss, prog.penalty, prog.auc, prog.nnz_w, prog.nrows], np.float64),
+              "fea_cnt": scal[:, 0], "w": scal[:, 1], "sqrt_g": scal[:, 2], "z": scal[:, 3],
+              "has_V": hasv.astype(np.float32), "V": V, "V_cg": cg}
+    os.makedirs(d, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(d, name + ".npy"), np.ascontiguousarray(a))
+
+
 def run_single(args, local_rank, full, sampler=None):
     """one configuration on one GPU.  Batches are the reader's raw CSR<uint64> (ids not localized): every step runs
     Localizer::Compact on the GPU, then the fused minibatch.  full: also e2e, localizer check, clocks."""
@@ -391,6 +422,8 @@ def run_single(args, local_rank, full, sampler=None):
     prog = E.read_progress()
     value = steps * B / (ms * 1e-3)
     st2 = E.table_stats()
+    if full and args.dump_outputs:
+        dump_outputs(E, args.dump_outputs, args, host[bi(warm + steps - 1)], prog)
 
     out = {"value": value, "ms_per_step": ms / steps, "gpu_launches": int(launches),
            "loss_per_example": prog.loss / max(prog.nrows, 1), "unique_keys_per_batch": int(U0),
@@ -593,6 +626,8 @@ def main():
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
+    if args.dump_outputs and (world > 1 or args.impl != "b200"):
+        sys.exit("--dump-outputs: only for the B200 arm on one GPU")
     if args.impl == "reference":
         return main_reference(args, rank, world)
     return main_b200(args, rank, world, local_rank)

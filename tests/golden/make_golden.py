@@ -1,18 +1,24 @@
 """Generate the committed golden fixtures from the UNMODIFIED reference.
 
-Run in the build container (needs /root/reference and `make -C oracle ref`):
+Needs the reference's sources, from which `make -C oracle ref` builds oracle/_ref (see oracle/Makefile):
 
-    python tests/golden/make_golden.py
+    python tests/golden/make_golden.py               # all three files
+    python tests/golden/make_golden.py ref_checks    # only ref_checks.npz
 
 Writes tests/golden/rcv1_100.npz  -- the reference's own 100-row fixture
 (/root/reference/tests/data, tests/README.md:5-7) as parsed by the reference's
 BatchReader + dmlc LibSVMParser (so values carry the reference's float parsing), and
 tests/golden/ref_outputs.npz -- outputs of the compiled reference (FMLoss, SGDUpdater,
-Localizer, SGDLearner) on that fixture and on small seeded synthetic batches.
-The GPU box has no /root/reference: tests read only these files.
+Localizer, SGDLearner) on that fixture and on small seeded synthetic batches, and
+tests/golden/ref_checks.npz -- the reference's outputs on the random inputs of
+tests/test_oracle_vs_ref.py and the batches its BatchReader yields in the cases of
+tests/test_host_cpp.py::test_shuffled_batches_equal_the_reference_reader.
+Tests read only these files: they need neither the reference nor oracle/_ref.
 """
 import os
+import subprocess
 import sys
+import tempfile
 
 import numpy as np
 
@@ -22,6 +28,26 @@ from oracle import oracle as O  # noqa: E402
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 REF_DATA = "/root/reference/tests/data"
+
+# one batch of the reference's BatchReader, read from the start in a fresh interpreter: it shuffles with rand(),
+# process-wide state.  Prints: batch index, rows, nnz, hash of the ids, hash of the labels, has values
+_REF_BATCH = r"""
+import sys
+sys.path.insert(0, sys.argv[1])
+from oracle import oracle as O
+path, part, nparts, bs, shuf, neg, which = sys.argv[2], int(sys.argv[3]), int(sys.argv[4]), int(sys.argv[5]), int(sys.argv[6]), float(sys.argv[7]), int(sys.argv[8])
+r = O.ref_read_batch(path, "libsvm", part, nparts, bs, shuf, neg, which)
+if r is None:
+    print("END")
+else:
+    off, lab, idx, val = r
+    hi = hl = 0
+    for x in idx.tolist():
+        hi = (hi * 1000003 + x) & 0xFFFFFFFFFFFFFFFF
+    for y in lab.tolist():
+        hl = (hl * 1000003 + (1 if y > 0 else 2)) & 0xFFFFFFFFFFFFFFFF
+    print(which, len(lab), len(idx), hi, hl, 1 if val is not None else 0)
+"""
 
 
 def synth_batches(seed, nbatch, B, max_nnz, id_space, with_values):
@@ -38,8 +64,7 @@ def synth_batches(seed, nbatch, B, max_nnz, id_space, with_values):
     return out
 
 
-def main():
-    O.build(ref=True)
+def fixtures():
     off, lab, idx, val = O.ref_read_batch(REF_DATA, "libsvm", 0, 1, 100)
     np.savez_compressed(os.path.join(HERE, "rcv1_100.npz"), offset=off, label=lab, index=idx, value=val)
 
@@ -127,5 +152,54 @@ def main():
     print("wrote", {k: getattr(v, "shape", None) for k, v in out.items()})
 
 
+def ref_checks():
+    sys.path.insert(0, os.path.join(ROOT, "tests"))
+    import test_host_cpp as H
+    import test_oracle_vs_ref as T
+    out = {}
+    # --- FMLoss / Localizer on random batches (test_oracle_vs_ref.py::test_loss_bit_exact) ---
+    for V_dim, valued in T.LOSS_CASES:
+        tag = f"loss_v{V_dim}_{int(valued)}_"
+        # the batch alone first: the weights loss_case draws after it need its number of distinct keys
+        rng = np.random.default_rng(V_dim * 2 + int(valued))
+        off, lab, idx, val = T.rand_batch(rng, 200, 30, 500, valued)
+        lidx, keys, cnt, _ = O.ref_localize(off, idx, val, lab)
+        off, lab, idx, val, W, w_pos, V_pos = T.loss_case(V_dim, valued, len(keys))
+        R = O.RefOracle(V_dim=V_dim)
+        pred = R.predict(off, lidx, val, W, w_pos, V_pos, lab)
+        out[tag + "lidx"], out[tag + "keys"], out[tag + "cnt"] = lidx, keys, cnt
+        out[tag + "pred"] = pred
+        out[tag + "grad"] = R.calc_grad(off, lidx, val, lab, W, pred, w_pos, V_pos)
+        out[tag + "objv"] = np.float32(R.evaluate(lab, pred))
+    # --- SGDUpdater trajectory (test_oracle_vs_ref.py::test_updater_trajectory_bit_exact) ---
+    R = O.RefOracle(**T.UPDATER_KW)
+    prog, seen = [], []
+    for step, (off, lab, idx, val) in enumerate(T.updater_batches()):
+        prog.append(R.sgd_step(off, idx, val, lab, *T.updater_flags(step)).copy())
+        seen.append(O.reverse_bytes_np(idx))
+    keys = np.unique(np.concatenate(seen))
+    out["updater_progress"], out["updater_keys"] = np.array(prog), keys
+    out["updater_vals"], out["updater_lens"] = R.get(keys)
+    # --- BatchReader shuffle + negative sampling (test_host_cpp.py::test_shuffled_batches_equal_the_reference_reader) ---
+    d = np.load(os.path.join(HERE, "rcv1_100.npz"))
+    with tempfile.TemporaryDirectory() as tmp:
+        data = os.path.join(tmp, "rcv1_100.libsvm")
+        H.write_libsvm(d, data)
+        for case in H.READER_CASES:
+            lines = []
+            for b in range(case[-1]):
+                r = subprocess.run([sys.executable, "-c", _REF_BATCH, ROOT, data] + [str(x) for x in case[:-1]] + [str(b)],
+                                   capture_output=True, text=True, check=True)
+                lines.append(r.stdout.strip().split("\n")[-1])
+            out[H.reader_tag(*case)] = np.array([x for x in lines if x != "END"])
+    np.savez_compressed(os.path.join(HERE, "ref_checks.npz"), **out)
+    print("wrote", {k: getattr(v, "shape", None) for k, v in out.items()})
+
+
 if __name__ == "__main__":
-    main()
+    O.build(ref=True)
+    which = sys.argv[1:] or ["fixtures", "ref_checks"]
+    if "fixtures" in which:
+        fixtures()
+    if "ref_checks" in which:
+        ref_checks()

@@ -193,7 +193,7 @@ def test_fused_shard_segment_capacity_is_reported():
     assert ei.value.code == capi.DFB_ERR_CAPACITY
 
 
-@pytest.mark.skipif(torch.cuda.device_count() < 2, reason="needs 2 GPUs (gpurun --gpus 2)")
+@pytest.mark.skipif(torch.cuda.device_count() < 2, reason="needs 2 GPUs")
 @pytest.mark.parametrize("big", [False, True])
 def test_fused_shard_two_gpus_one_process_vs_oracle_simulation(big):
     """two engines on two devices inside ONE process, driven by ONE host thread (peer access instead of CUDA IPC; the
@@ -250,7 +250,7 @@ def _worker(rank, world, port, out):
     dist.destroy_process_group()
 
 
-@pytest.mark.skipif(torch.cuda.device_count() < 2, reason="needs 2 GPUs (gpurun --gpus 2)")
+@pytest.mark.skipif(torch.cuda.device_count() < 2, reason="needs 2 GPUs")
 def test_fused_shard_two_gpus_ipc_vs_oracle_simulation(tmp_path):
     import torch.multiprocessing as mp
     world = 2

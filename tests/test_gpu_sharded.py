@@ -115,7 +115,7 @@ def _worker(rank, world, port, out, p2p):
     dist.destroy_process_group()
 
 
-@pytest.mark.skipif(torch.cuda.device_count() < 2, reason="needs 2 GPUs (gpurun --gpus 2)")
+@pytest.mark.skipif(torch.cuda.device_count() < 2, reason="needs 2 GPUs")
 @pytest.mark.parametrize("p2p", [False, True])
 def test_two_gpu_nccl_sharded_vs_oracle_simulation(tmp_path, p2p):
     import torch.multiprocessing as mp

@@ -9,6 +9,7 @@ import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 BIN = os.path.join(ROOT, "difacto_b200", "host", "bin")
+GOLDEN_REF_CHECKS = os.path.join(ROOT, "tests", "golden", "ref_checks.npz")
 
 
 @pytest.fixture(scope="session")
@@ -21,15 +22,19 @@ def host_bin():
     return BIN
 
 
-@pytest.fixture(scope="session")
-def libsvm_fixture(tmp_path_factory, rcv1):
+def write_libsvm(rcv1, path):
     """the reference's 100-row fixture as libsvm text (%.9g round-trips float32 exactly)"""
-    path = tmp_path_factory.mktemp("data") / "rcv1_100.libsvm"
     off, lab, idx, val = rcv1["offset"], rcv1["label"], rcv1["index"], rcv1["value"]
     with open(path, "w") as f:
         for r in range(len(lab)):
             feats = " ".join(f"{int(idx[j])}:{val[j]:.9g}" for j in range(int(off[r]), int(off[r + 1])))
             f.write(f"{int(lab[r])} {feats}\n")
+
+
+@pytest.fixture(scope="session")
+def libsvm_fixture(tmp_path_factory, rcv1):
+    path = tmp_path_factory.mktemp("data") / "rcv1_100.libsvm"
+    write_libsvm(rcv1, path)
     return str(path)
 
 
@@ -41,44 +46,25 @@ def test_host_unit_cases_cpu(host_bin, libsvm_fixture):
     assert "BatchReader.StreamedChunks" in out.stdout
 
 
-_REF_BATCH = r"""
-import sys
-sys.path.insert(0, sys.argv[1])
-from oracle import oracle as O
-path, part, nparts, bs, shuf, neg, which = sys.argv[2], int(sys.argv[3]), int(sys.argv[4]), int(sys.argv[5]), int(sys.argv[6]), float(sys.argv[7]), int(sys.argv[8])
-r = O.ref_read_batch(path, "libsvm", part, nparts, bs, shuf, neg, which)
-if r is None:
-    print("END")
-else:
-    off, lab, idx, val = r
-    hi = hl = 0
-    for x in idx.tolist():
-        hi = (hi * 1000003 + x) & 0xFFFFFFFFFFFFFFFF
-    for y in lab.tolist():
-        hl = (hl * 1000003 + (1 if y > 0 else 2)) & 0xFFFFFFFFFFFFFFFF
-    print(which, len(lab), len(idx), hi, hl, 1 if val is not None else 0)
-"""
+# (part, nparts, batch_size, shuffle window, negative sampling, batches); the reference's batches of every case are
+# stored in tests/golden/ref_checks.npz (tests/golden/make_golden.py)
+READER_CASES = [(0, 1, 10, 30, 1.0, 5), (1, 2, 7, 21, 0.5, 4)]
 
 
-@pytest.mark.parametrize("part,nparts,bs,shuf,neg,nb", [(0, 1, 10, 30, 1.0, 5), (1, 2, 7, 21, 0.5, 4)])
+def reader_tag(part, nparts, bs, shuf, neg, nb):
+    return f"reader_{part}_{nparts}_{bs}_{shuf}_{neg:g}_{nb}"
+
+
+@pytest.mark.parametrize("part,nparts,bs,shuf,neg,nb", READER_CASES)
 def test_shuffled_batches_equal_the_reference_reader(host_bin, libsvm_fixture, part, nparts, bs, shuf, neg, nb):
     """shuffle window + negative down-sampling: the host BatchReader in its reference order (libstdc++'s
     std::random_shuffle on rand(), persistent permutation, rand_r seed 0: src/reader/batch_reader.cc:8-78) yields the
-    very batches of the reference's BatchReader, row for row.  rand() is process-wide state, so every batch of the
-    compiled reference (oracle/_ref) is read in a fresh interpreter that replays the reader from the start."""
-    from oracle import oracle as O
-    if not O.have_ref():
-        pytest.skip("the compiled reference (oracle/_ref) is not available")
+    very batches of the reference's BatchReader, row for row: per batch its index, rows, nnz, a hash of the ids, a hash
+    of the labels and whether it carries values, as the compiled reference printed them."""
     ours = subprocess.run([os.path.join(host_bin, "batch_dump"), libsvm_fixture, str(part), str(nparts), str(bs), str(shuf),
                            str(neg), str(nb), "reference"], capture_output=True, text=True)
     assert ours.returncode == 0, ours.stderr
-    ref = []
-    for b in range(nb):
-        out = subprocess.run([sys.executable, "-c", _REF_BATCH, ROOT, libsvm_fixture, str(part), str(nparts), str(bs), str(shuf),
-                              str(neg), str(b)], capture_output=True, text=True)
-        assert out.returncode == 0, out.stderr
-        ref.append(out.stdout.strip().split("\n")[-1])
-    ref = [r for r in ref if r != "END"]
+    ref = [str(r) for r in np.load(GOLDEN_REF_CHECKS)[reader_tag(part, nparts, bs, shuf, neg, nb)]]
     assert len(ref) >= 3
     assert ours.stdout.strip().split("\n") == ref
     # the seeded order (num_gpus > 1: concurrent readers) is a different permutation of the same rows
@@ -294,7 +280,7 @@ def test_cli_two_gpus_sharded_store(host_bin, tmp_path):
     and a reloaded model must reproduce the validation loss it was saved with."""
     import torch
     if torch.cuda.device_count() < 2:
-        pytest.skip("needs 2 GPUs (gpurun --gpus 2)")
+        pytest.skip("needs 2 GPUs")
     exe = os.path.join(host_bin, "difacto_b200")
     data, val = str(tmp_path / "train.libsvm"), str(tmp_path / "val.libsvm")
     _synthetic_libsvm(data, 4000, 1)
